@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """Benchmark of the batched differential-IK hot path (BASELINE.json metric).
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]
 
 A "step" is one ``solve_ik`` pass over one batch of B = 65536 UR5 instances per
 GPU (FrameTask(tool0) + PostureTask + default limits, examples/arm_ur5.py).
@@ -35,6 +35,26 @@ UNIT = "IK steps/s"
 BYTES_PER_STEP = 96  # q 24 B + frame target 48 B read, v 24 B written (BASELINE.md section 4)
 L2_BYTES = 126 * 1024 * 1024
 GRAPH_CHUNK = 512    # launches per captured graph when K is larger than this
+DUMP_LIMIT = 64_000_000  # bytes --dump-outputs may write in all, .npy headers included
+
+
+def dump_outputs(out_dir, arrays):
+    """``--dump-outputs``: every array of ``arrays`` (name -> [B, ...] over the same B instances)
+    as ``out_dir/<name>.npy``, float64 kept, anything else as float32.  When they would exceed
+    DUMP_LIMIT, every array keeps the same fixed, seeded sample of instances (ascending), and the
+    instance indices are written as ``instance.npy``."""
+    arrays = {k: a if a.dtype == np.float64 else a.astype(np.float32) for k, a in arrays.items()}
+    budget = DUMP_LIMIT - 256 * (len(arrays) + 1)  # room for the .npy headers (128 bytes each here)
+    total = sum(a.nbytes for a in arrays.values())
+    if total > budget:
+        B = next(iter(arrays.values())).shape[0]
+        n = budget * B // (total + 8 * B)  # rows that fit together with their float64 index
+        rows = np.sort(np.random.default_rng(0).choice(B, size=n, replace=False))
+        arrays = {k: a[rows] for k, a in arrays.items()}
+        arrays["instance"] = rows.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a))
 
 
 def committed_traffic():
@@ -242,8 +262,10 @@ def run_reference_arm(args):
         arm.step(threads)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        arm.step(threads)
+        _, v, st = arm.step(threads)
     wall = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"v": v, "status": st})
     value = args.batch * args.steps / wall
     one = min(arm.step(1)[0] for _ in range(2))
     one_core = args.batch / one
@@ -753,6 +775,8 @@ def run_gpu_arm(args):
 
     with ClockSampler(local) as clocks:
         ms, region_ms = timed_regions(graphed.run if graphed is not None else run_eager, args.regions)
+        last = (args.steps - 1) % NBUF  # the buffer set the last timed step wrote
+        outputs = {"v": vs[last].cpu().numpy(), "status": ss[last].cpu().numpy()} if args.dump_outputs else None
         # keep the GPU under the same load a little longer so the sampler sees it
         t_end = time.time() + 0.5
         while time.time() < t_end:
@@ -946,6 +970,8 @@ def run_gpu_arm(args):
         if not args.no_cpu and world == 1:
             os.sched_setaffinity(0, full_affinity)  # the CPU arm gets every core again
             line["cpu_baseline"] = cpu_baseline_block(B)
+        if outputs is not None:
+            dump_outputs(args.dump_outputs, outputs)
         if real_stdout is not None:
             os.write(real_stdout, (json.dumps(line) + "\n").encode())
         else:
@@ -973,7 +999,13 @@ def main():
     ap.add_argument("--no-numa-bind", action="store_true")
     ap.add_argument("--e2e-sets", type=int, default=2, help="pinned host buffer sets the e2e steps rotate over")
     ap.add_argument("--e2e-streams", type=int, default=2, help="caller streams the e2e steps alternate over (2: consecutive calls pipeline through the library's two staging sets)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write v and status of the last one (rank 0's shard) as DIR/<name>.npy; "
+                         "--impl ours dumps input set (steps - 1) %% nbuf, --impl reference its one workload, so the two "
+                         "dump the same instances only when steps %% nbuf == 1")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference_arm(args)

@@ -1,8 +1,8 @@
 #!/usr/bin/env python3
 """Freeze outputs of the REFERENCE's own Pink-layer Python under tests/golden/ref_pink_layer_*.npz.
 
-Runs only in the build container: it imports the UNMODIFIED package ``pink`` from
-``/root/reference`` with the two name shims of ``oracle/refshim`` (``pinocchio``,
+It imports the UNMODIFIED package ``pink`` of the reference, byte-compiled by ``build()`` into
+``oracle/_ref/pink`` (oracle/ref_build.py), with the two name shims of ``oracle/refshim`` (``pinocchio``,
 ``qpsolvers``: oracle-backed stand-ins, see oracle/refshim/README.md) in front of it, because
 the real third-party modules are neither installed nor installable here.  For every seeded
 case it builds the reference's task / limit / barrier OBJECTS, then calls the reference's
@@ -13,7 +13,7 @@ velocity and every task's ``compute_error`` / ``compute_jacobian``.
     python scripts/make_reference_golden.py --check  # re-runs the reference and compares with the committed files
 
 ``tests/test_reference_pink_layer_golden.py`` compares the oracle's own assembly (and the
-kernels) with these files; nothing under tests/ imports /root/reference or the shims.
+kernels) with these files; nothing under tests/ imports the reference or the shims.
 
 What the fixtures pin and what they do not: oracle/refshim/README.md.
 """
@@ -21,8 +21,8 @@ import os
 import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REFERENCE = "/root/reference"
-# order matters: /root/reference also has a package called `tests`
+REFERENCE = os.path.join(ROOT, "oracle", "_ref")
+# order matters: the staged reference also has a package called `tests`
 sys.path[:0] = [os.path.join(ROOT, "oracle", "refshim"), ROOT, REFERENCE]
 
 import numpy as np  # noqa: E402
@@ -193,7 +193,7 @@ def run_case(name):
 def run_example(name):
     """Closed loop of a reference example on the URDF the reference vendors for it."""
     fname, steps = cases.EXAMPLE_LOOPS[name]
-    robot = pin.RobotWrapper(pin.pinocchio_like_limits(pin.load_urdf(os.path.join(REFERENCE, "examples", "robots", fname)).model))
+    robot = pin.RobotWrapper(pin.pinocchio_like_limits(pin.load_urdf(os.path.join(GOLDEN, "reference_robots", fname)).model))
     q, v = cases.run_example_loop(name, pink, robot, steps)
     path = os.path.join(GOLDEN, f"ref_example_{name}.npz")
     if CHECK:

@@ -1,9 +1,10 @@
 #!/usr/bin/env python3
-"""Run the REFERENCE's own test files (/root/reference/tests, unmodified) against the
-reference's own Pink-layer code, with the oracle standing in for the third-party primitives.
+"""Run the REFERENCE's own test files (unmodified, byte-compiled by ``build()`` into
+``oracle/_ref/tests``, see oracle/ref_build.py) against the reference's own Pink-layer code
+(``oracle/_ref/pink``), with the oracle standing in for the third-party primitives.
 
-Build container only (``/root/reference`` does not travel).  ``oracle/refshim`` supplies the
-module names ``pinocchio``, ``qpsolvers`` and ``robot_descriptions`` (oracle-backed stand-ins,
+``oracle/refshim`` supplies the module names ``pinocchio``, ``qpsolvers`` and
+``robot_descriptions`` (oracle-backed stand-ins,
 see oracle/refshim/README.md); robots the reference clones from the network are replaced by
 offline stand-ins of the same class (oracle/refshim/robot_descriptions/loaders/pinocchio.py)
 or the test is skipped.  Every known-answer test of the reference that does not depend on the
@@ -23,7 +24,7 @@ import subprocess
 import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REFERENCE = "/root/reference"
+REFERENCE = os.path.join(ROOT, "oracle", "_ref")
 OUT_OF_SCOPE = {
     "test_manipulability_task.py": "ManipulabilityTask is out of scope (SURVEY section 2)",
     "test_rolling_task.py": "wheel tasks are out of scope (SURVEY section 2)",
@@ -68,8 +69,11 @@ def main():
     expected = PRODUCT_EXPECTED_FAILURES if product else EXPECTED_FAILURES
     env = dict(os.environ)
     env["PYTHONPATH"] = os.pathsep.join([os.path.join(ROOT, "oracle", "refshim"), ROOT, REFERENCE])
-    cmd = [sys.executable, "-m", "pytest", os.path.join(REFERENCE, "tests"), "-p", "no:cacheprovider", "-q", "-rA", "-W", "ignore",
-           "--tb=line"] + [f"--ignore={os.path.join(REFERENCE, 'tests', f)}" for f in OUT_OF_SCOPE]
+    # the staged test modules are sourceless: pytest's check that a module came from the .py file
+    # it collected does not apply to them
+    env["PY_IGNORE_IMPORTMISMATCH"] = "1"
+    cmd = [sys.executable, "-m", "pytest", os.path.join(REFERENCE, "tests"), "-p", "oracle.ref_build", "-p", "no:cacheprovider",
+           "-q", "-rA", "-W", "ignore", "--tb=line"] + [f"--ignore={os.path.join(REFERENCE, 'tests', f + 'c')}" for f in OUT_OF_SCOPE]
     if product:
         cmd += ["-p", "tests.refalias_plugin", "--import-mode=importlib"]
     res = subprocess.run(cmd, cwd="/tmp", env=env, capture_output=True, text=True)
@@ -78,17 +82,17 @@ def main():
     for ln in lines:
         m = re.match(r"(PASSED|FAILED|SKIPPED|ERROR)\s+(.*)", ln)
         if m:
-            outcomes.append((m.group(1), m.group(2).replace("../root/reference/tests/", "").replace("../root/reference/", "")))
+            outcomes.append((m.group(1), re.sub(r"^(\[\d+\] )?\S*?tests/(test_\w+)\.pyc?", r"\1\2.py", m.group(2))))
     summary = next((ln for ln in reversed(lines) if re.search(r"\d+ passed", ln)), "no summary")
     unexpected = [t for o, t in outcomes if o in ("FAILED", "ERROR") and not any(t.startswith(k) for k in expected)]
     with open(record, "w") as fh:
         if product:
-            fh.write("# The reference's own tests (/root/reference/tests, unmodified) against THIS package: the module name\n"
+            fh.write("# The reference's own tests (unmodified, staged in oracle/_ref) against THIS package: the module name\n"
                      "# `pink` is bound to pink_b200 (tests/refalias_plugin.py), the engine is the host build of the CUDA kernel\n"
                      "# bodies (fp32), pinocchio / qpsolvers / robot_descriptions are the stand-ins of oracle/refshim.  Made by\n"
                      "# scripts/run_reference_tests.py --product in the build container.  NOT a GPU capture.\n")
         else:
-            fh.write("# The reference's own tests (/root/reference/tests, unmodified) over its own Pink-layer code, with\n"
+            fh.write("# The reference's own tests (unmodified, staged in oracle/_ref) over its own Pink-layer code, with\n"
                      "# oracle/refshim standing in for pinocchio / qpsolvers / robot_descriptions.  Made by\n"
                      "# scripts/run_reference_tests.py in the build container.  NOT a GPU capture.\n")
         fh.write(f"# pytest summary: {summary.strip('= ')}\n")

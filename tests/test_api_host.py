@@ -16,7 +16,7 @@ from pink_b200.solve_ik import describe_problem
 from pink_b200.utils import VectorSpace, custom_configuration_vector, get_joint_idx, get_root_joint_dim
 from tests import helpers
 
-REF_ROBOTS = "/root/reference/examples/robots"
+REF_ROBOTS = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_robots")
 
 
 def test_ur5_model_dimensions_and_zero_pose():
@@ -46,7 +46,6 @@ def test_free_flyer_models_follow_pinocchio_conventions():
         assert len(ConfigurationLimit(model).indices) == nj
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_ROBOTS), reason="reference checkout not present")
 @pytest.mark.parametrize("fname,nq", [("double_pendulum.urdf", 2), ("planar_2dof.urdf", 2), ("simple_pendulum.urdf", 1)])
 def test_urdf_loader_on_the_reference_fixtures(fname, nq):
     robot = load_urdf(os.path.join(REF_ROBOTS, fname))

@@ -128,10 +128,9 @@ def test_cuda_library_matches_the_reference_velocities(name):
 
 # ---- closed loops of two reference examples (tests/golden/ref_example_*.npz) ---------------------
 def _example_robot(fname):
-    from pink_b200.model import RobotWrapper, model_from_urdf_string
-    from tests.test_reference_urdf_closed_forms import SKELETONS  # proven identical to the reference's URDF files
+    from pink_b200.model import load_urdf
 
-    return RobotWrapper(model_from_urdf_string(SKELETONS[fname]))
+    return load_urdf(os.path.join(GOLDEN, "reference_robots", fname))
 
 
 def _check_example(name, q, v):

@@ -1,4 +1,5 @@
-"""Build container only (skipped where /root/reference does not exist, i.e. on the GPU box):
+"""The reference's own code, byte-compiled by ``build()`` into oracle/_ref (oracle/ref_build.py);
+skipped where no build has staged it:
 
 * the reference's own test files run, unmodified, over its own Pink-layer code with the oracle
   standing in for the third-party primitives (scripts/run_reference_tests.py; committed record:
@@ -15,8 +16,10 @@ import sys
 
 import pytest
 
+from oracle import ref_build
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-needs_reference = pytest.mark.skipif(not os.path.isdir("/root/reference/pink"), reason="/root/reference is not mounted here")
+needs_reference = pytest.mark.skipif(not ref_build.staged(), reason="no reference staged in oracle/_ref by build()")
 
 
 @needs_reference

@@ -1,9 +1,10 @@
 """Pins the URDF loader, forward kinematics and LOCAL frame Jacobians to files the REFERENCE
-holds: the three robots vendored under /root/reference/examples/robots (used by
+holds: the three robots it vendors under examples/robots (used by
 examples/double_pendulum.py:28-36, planar_2dof_manipulability.py:35-43,
-one_dof_configuration_limit.py:44-53).  Their kinematics has closed forms, written out below
-by hand from the URDF numbers - independent of the oracle, of the model loader and of the
-kernels - so that all three are tied to reference-held inputs:
+one_dof_configuration_limit.py:44-53), stored unmodified in tests/golden/reference_robots/.
+Their kinematics has closed forms, written out below by hand from the URDF numbers -
+independent of the oracle, of the model loader and of the kernels - so that all three are
+tied to reference-held inputs:
 
 * simple_pendulum: joint about x at the origin, tip 0.25 m up the body
       p = (0, -0.25 sin q, 0.25 cos q),  R = Rx(q)
@@ -22,30 +23,7 @@ import os
 import numpy as np
 import pytest
 
-REF_ROBOTS = "/root/reference/examples/robots"
-needs_reference = pytest.mark.skipif(not os.path.isdir(REF_ROBOTS), reason="reference checkout not present")
-
-# Kinematic skeletons of the same three robots (joint origins / axes / limits as in the
-# reference files, nothing else) for the GPU box, where /root/reference does not exist; the
-# CPU suite checks that they describe the same models as the reference URDFs.
-SKELETONS = {
-    "simple_pendulum.urdf": """<robot name="simple_pendulum"><link name="base"/><link name="body"/><link name="tip"/>
-      <joint name="joint" type="revolute"><origin xyz="0 0 0"/><parent link="base"/><child link="body"/>
-        <axis xyz="1 0 0"/><limit lower="0.0" upper="6.28" velocity="1.0"/></joint>
-      <joint name="fixed_tip" type="fixed"><origin xyz="0 0 0.25"/><parent link="body"/><child link="tip"/></joint></robot>""",
-    "double_pendulum.urdf": """<robot name="double_pendulum"><link name="base_link"/><link name="link1"/><link name="link2"/><link name="link3"/>
-      <joint name="joint1" type="revolute"><origin xyz="0.025 0 0"/><parent link="base_link"/><child link="link1"/>
-        <axis xyz="1 0 0"/><limit lower="0" upper="0" velocity="0"/></joint>
-      <joint name="joint2" type="revolute"><origin xyz="0.0125 0 0.1"/><parent link="link1"/><child link="link2"/>
-        <axis xyz="1 0 0"/><limit lower="0" upper="0" velocity="0"/></joint>
-      <joint name="joint3" type="fixed"><origin xyz="0 0 0.2"/><parent link="link2"/><child link="link3"/></joint></robot>""",
-    "planar_2dof.urdf": """<robot name="planar_2dof"><link name="base_link"/><link name="link1"/><link name="link2"/><link name="end_effector"/>
-      <joint name="joint1" type="revolute"><origin xyz="0.025 0 0"/><parent link="base_link"/><child link="link1"/>
-        <axis xyz="0 0 1"/><limit lower="-3.14159" upper="3.14159" velocity="2"/></joint>
-      <joint name="joint2" type="revolute"><origin xyz="0.2 0 0"/><parent link="link1"/><child link="link2"/>
-        <axis xyz="0 0 1"/><limit lower="-3.14159" upper="3.14159" velocity="2"/></joint>
-      <joint name="end_effector_joint" type="fixed"><origin xyz="0.2 0 0"/><parent link="link2"/><child link="end_effector"/></joint></robot>""",
-}
+REF_ROBOTS = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_robots")
 
 
 def Rx(a):
@@ -102,7 +80,6 @@ def _configs(nq, n=40, seed=3):
     return rng.uniform(-3.0, 3.0, size=(n, nq))
 
 
-@needs_reference
 @pytest.mark.parametrize("fname,nq", ROBOTS)
 def test_oracle_fk_and_local_jacobian_match_the_closed_forms(fname, nq):
     from oracle import kinematics as okin
@@ -119,7 +96,6 @@ def test_oracle_fk_and_local_jacobian_match_the_closed_forms(fname, nq):
         np.testing.assert_allclose(okin.frame_jacobian_local(table, fk, f)[i], J, atol=1e-12)
 
 
-@needs_reference
 @pytest.mark.parametrize("fname,nq", ROBOTS)
 def test_host_build_of_the_kernels_matches_the_closed_forms(fname, nq):
     from tests.hostsim import HostSim
@@ -138,7 +114,6 @@ def test_host_build_of_the_kernels_matches_the_closed_forms(fname, nq):
         np.testing.assert_allclose(Jh[i], J, atol=2e-6)
 
 
-@needs_reference
 @pytest.mark.parametrize("fname,nq", ROBOTS)
 def test_limits_read_from_the_reference_urdfs(fname, nq):
     robot, table = _load(fname)
@@ -155,7 +130,6 @@ def test_limits_read_from_the_reference_urdfs(fname, nq):
         assert len(VelocityLimit(robot.model).indices) == 0
 
 
-@needs_reference
 @pytest.mark.parametrize("fname,nq", ROBOTS)
 def test_frame_task_error_and_jacobian_from_closed_forms(fname, nq):
     """FrameTask.compute_error / compute_jacobian (pink/tasks/frame_task.py:176-226) evaluated
@@ -197,36 +171,14 @@ def test_frame_task_error_and_jacobian_from_closed_forms(fname, nq):
     np.testing.assert_allclose(Jt[0], Jfd, atol=1e-6)
 
 
-@needs_reference
-@pytest.mark.parametrize("fname,nq", ROBOTS)
-def test_skeletons_describe_the_reference_models(fname, nq):
-    from pink_b200.model import model_from_urdf_string
-
-    ref = _load(fname)[1]
-    sk = model_from_urdf_string(SKELETONS[fname]).table()
-    for field in ("parent", "jtype", "joint_R", "joint_p", "axis", "q_min", "q_max", "v_max", "frame_body"):
-        a, b = np.asarray(getattr(ref, field), dtype=float), np.asarray(getattr(sk, field), dtype=float)
-        if field == "frame_body":  # the skeleton has the same link frames in the same order
-            assert list(ref.frame_names) == list(sk.frame_names)
-        np.testing.assert_allclose(a, b, atol=1e-15, err_msg=field)
-
-
 @pytest.mark.gpu
 @pytest.mark.parametrize("fname,nq", ROBOTS)
 def test_cuda_library_matches_the_closed_forms(fname, nq):
     import torch
 
     from pink_b200.engine import get_engine
-    from pink_b200.model import model_from_urdf_string
 
-    model = model_from_urdf_string(SKELETONS[fname])
-    robot, table = None, model.table()
-
-    class _R:  # same shape as the loader's return value
-        pass
-
-    robot = _R()
-    robot.model = model
+    robot, table = _load(fname)
     eng = get_engine(robot.model)
     q = _configs(nq).astype(np.float32)
     q_d = torch.as_tensor(q, device=eng.device)
